@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2|C3|C4|C5|P360]     # this repo's CUDA path
     python bench.py --impl reference [...]                                              # the reference algorithm on the host CPU cores
+    python bench.py --dump-outputs DIR [...]                                            # + the last timed step's results as DIR/<key>.npy
 
 A step is one pass of the hot path over one batch of synthetic input.  Configurations (BASELINE.json `configs`, SURVEY.md 8d):
   C2 (default, the configuration the metric is quoted on): ``Paramnet-360Cities-edina-centered``, 32 x 640x480 per GPU
@@ -62,6 +63,7 @@ def parse():
     ap.add_argument("--micro-batch", type=int, default=32, help="images per micro-batch of the gather-inclusive multi-GPU leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile-passes", action="store_true", help="skip the roofline / per-kernel passes (A/B timing runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step (rank 0's shard) as DIR/<key>.npy")
     return ap.parse_args()
 
 
@@ -191,8 +193,10 @@ def run_reference(args, rank):
     per_step = []
     for _ in range(args.steps):
         t = time.perf_counter()
-        om.inference_batch(sd, cfg["version"], imgs)
+        res = om.inference_batch(sd, cfg["version"], imgs)
         per_step.append(time.perf_counter() - t)
+    if args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)
     dt = sum(per_step)
     v = n * args.steps / dt
     sample = (f"{n} of the {B} images of the step's batch per step ({args.steps} steps, 1 warm-up on the same sample), torch CPU fp32, "
@@ -238,9 +242,9 @@ class Bench:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return t.item()
 
-    def resident_leg(self, imgs, steps, warmup, sampler=None, trace=False):
+    def resident_leg(self, imgs, steps, warmup, sampler=None, trace=False, dump_dir=None):
         """K steps with the inputs already in HBM: flush L2, pf_forward on the staged blob.  Returns (ms of the timed region on this
-        rank, kernel launches, host enqueue ms per step)."""
+        rank, kernel launches, host enqueue ms per step).  ``dump_dir``: write the last step's results there (dump_outputs)."""
         torch = self.torch
         B = len(imgs)
         heights, widths = [im.shape[0] for im in imgs], [im.shape[1] for im in imgs]
@@ -268,6 +272,8 @@ class Bench:
             while not e1.query() and len(sampler.rows) < 64:
                 sampler.sample()
         self.barrier()
+        if dump_dir is not None:
+            dump_outputs(self.model.assemble_raw(out), dump_dir)
         del out
         return e0.elapsed_time(e1), self.L.pf_kernel_launch_count() - l0, host_ms, (blob, offsets, heights, widths)
 
@@ -357,6 +363,28 @@ class Bench:
         wall_ms = (time.perf_counter() - tw) * 1000
         pending.clear()
         return max(f0.elapsed_time(f1), wall_ms), h2d_bytes, d2h_bytes
+
+
+DUMP_MAX_ELEMENTS = 1 << 21   # per key (8 MiB of float32): the four field keys of a step stay below 64 MB in all
+
+
+def dump_outputs(results, dirname):
+    """The result dictionaries of ``inference_batch`` (what a caller of the timed path receives) as DIR/<key>.npy, float32,
+    one file per tensor key with the images stacked on a leading axis (the scalar camera parameters become [n] vectors).  A key
+    of more than DUMP_MAX_ELEMENTS elements is written flattened and sampled: the elements at sorted flat indices drawn with a
+    fixed seed from its size alone, so that the files of two builds run with the same arguments compare element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(dirname, exist_ok=True)
+    for key, v in results[0].items():
+        if isinstance(v, str):
+            continue
+        t = torch.stack([r[key] for r in results])
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), DUMP_MAX_ELEMENTS))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(dirname, key + ".npy"), t.float().cpu().numpy())
 
 
 def roofline_objects(args, B, prof, prof_ms, ms, per_kernel, heights, widths, peaks, write_peak=None):
@@ -581,7 +609,8 @@ def main():
     gc.disable()
 
     # ---------------- leg 1: inputs resident in HBM ("value") ------------------------------------------------
-    ms, launches, host_ms, staged = b.resident_leg(imgs, args.steps, args.warmup, sampler)
+    ms, launches, host_ms, staged = b.resident_leg(imgs, args.steps, args.warmup, sampler,
+                                                   dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop()
     ms_max = b.max_over_ranks(ms)
     value = world * B * args.steps / (ms_max / 1000.0)

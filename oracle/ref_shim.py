@@ -12,9 +12,8 @@ The reference needs ``timm``, ``yacs``, ``omegaconf``, ``matplotlib``, ``equilib
 * ``matplotlib*``, ``equilib`` (``__version__ == "0.3.0"`` is asserted in utils/panocam.py:8),
   ``imageio``                      -> empty modules
 
-Nothing here is imported by the product package.  ``/root/reference`` does not exist on the
-GPU box, so only the golden generator (tests/golden/make_golden.py) and the CPU-side
-"oracle == reference" tests (skipped when the reference is absent) call ``load_reference``.
+Nothing here is imported by the product package or by the tests: only the golden generators
+(tests/golden/make_golden*.py) call ``load_reference``, and the tests compare with what they stored.
 """
 import os
 import sys

@@ -32,27 +32,58 @@ def rel_err(a, b):
     return ((a - b).abs().max() / b.abs().max().clamp_min(1e-30)).item()
 
 
+def byte_planes(a):
+    """A float64 array as its 8 byte planes (uint8 [8, numel]): smooth fields stored this way compress about 20 % better."""
+    return np.ascontiguousarray(a, np.float64).view(np.uint8).reshape(-1, 8).T.copy()
+
+
+def from_byte_planes(p, shape):
+    return np.ascontiguousarray(p.T).view(np.float64).reshape(tuple(shape))
+
+
 def compare_with_golden(version, results, tol, check_stats=True, skip_keys=()):
     """Compare a list of result dicts (one per golden image) with the stored reference outputs.
     Returns {key: worst relative error}."""
     m, g = load_golden(version)
     worst = {}
     for i, res in enumerate(results):
-        assert list(res.keys()) == m["versions"][version]["keys"][i], (list(res.keys()), m["versions"][version]["keys"][i])
-        for k, v in res.items():
-            if isinstance(v, str):
-                assert v == "deg"
-                continue
-            if k in skip_keys:
-                continue
-            v = v.detach().cpu().float()
-            assert tuple(v.shape) == tuple(g[f"{i}/{k}/shape"]), (k, v.shape)
-            st = m["logit_stride"] if (v.ndim == 3 and v.shape[0] > 3) else m["stride"]
-            sub = v[..., ::st, ::st] if v.ndim >= 2 else v
-            e = rel_err(sub, g[f"{i}/{k}"])
+        w = compare_result(res, g, f"{i}/", m["versions"][version]["keys"][i], m["stride"], m["logit_stride"], tol,
+                           f"{version} img{i}", check_stats, skip_keys)
+        for k, e in w.items():
             worst[k] = max(worst.get(k, 0.0), e)
-            assert e <= tol, f"{version} img{i} {k}: rel err {e:.3g} > {tol}"
-            if check_stats:
-                s, sa, n = g[f"{i}/{k}/stats"]
-                assert abs(v.double().abs().sum().item() - sa) <= tol * max(sa, 1e-30) * 4, (k, "abs-sum checksum")
+    return worst
+
+
+def subsample(v, stride, logit_stride, edges=False):
+    """The rows and columns of ``v`` (torch, [..., H, W]) at ``stride`` (``logit_stride`` for logit tensors); ``edges`` adds
+    the last row and column when the stride misses them."""
+    if v.ndim < 2:
+        return v
+    st = logit_stride if (v.ndim == 3 and v.shape[0] > 3) else stride
+
+    def index(n):
+        i = list(range(0, n, st))
+        return i + [n - 1] if edges and i[-1] != n - 1 else i
+    return v[..., index(v.shape[-2]), :][..., index(v.shape[-1])]
+
+
+def compare_result(res, g, prefix, keys, stride, logit_stride, tol, label, check_stats=True, skip_keys=(), edges=False):
+    """Compare one result dict with reference outputs stored under ``prefix`` in ``g``: each tensor as a sub-sample
+    (``subsample``) plus its float64 (sum, abs-sum, numel).  Returns {key: relative error}."""
+    assert list(res.keys()) == list(keys), (list(res.keys()), list(keys))
+    worst = {}
+    for k, v in res.items():
+        if isinstance(v, str):
+            assert v == "deg"
+            continue
+        if k in skip_keys:
+            continue
+        v = v.detach().cpu().float()
+        assert tuple(v.shape) == tuple(g[f"{prefix}{k}/shape"]), (k, v.shape)
+        e = rel_err(subsample(v, stride, logit_stride, edges), g[f"{prefix}{k}"])
+        worst[k] = e
+        assert e <= tol, f"{label} {k}: rel err {e:.3g} > {tol}"
+        if check_stats:
+            s, sa, n = g[f"{prefix}{k}/stats"]
+            assert abs(v.double().abs().sum().item() - sa) <= tol * max(sa, 1e-30) * 4, (k, "abs-sum checksum")
     return worst

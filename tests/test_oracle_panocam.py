@@ -1,5 +1,5 @@
 """CPU: the oracle's camera-parameters -> field restatement (oracle/panocam.py) against golden vectors produced by the
-unmodified reference (tests/golden/panocam.npz, make_golden_panocam.py), live against the reference where it exists, and
+unmodified reference (tests/golden/panocam.npz, make_golden_panocam.py; reference_checks.npz, make_golden_reference_checks.py), and
 the host-side closed form of general_vfov_to_focal against the reference's fsolve formulation."""
 import ctypes
 import os
@@ -7,8 +7,8 @@ import os
 import numpy as np
 import pytest
 
+from golden_util import from_byte_planes
 from oracle import panocam as op
-from oracle.ref_shim import load_reference, reference_available
 
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "panocam.npz"))
 
@@ -28,17 +28,14 @@ def test_oracle_matches_reference_golden(i):
     assert np.allclose(np.linalg.norm(up, axis=2), 1.0, atol=1e-12)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference is not present on this machine")
 def test_oracle_matches_live_reference():
-    load_reference()
-    from perspective2d.utils.panocam import PanoCam
-    rs = np.random.RandomState(3)
-    for _ in range(6):
-        f, el, roll = rs.uniform(0.3, 2.0), rs.uniform(-1.4, 1.4), rs.uniform(-3.1, 3.1)
-        cx, cy = rs.uniform(-0.3, 0.3, 2)
-        w, h = int(rs.randint(2, 60)), int(rs.randint(2, 60))
-        assert np.abs(op.get_up_general(f, w, h, el, roll, cx, cy) - PanoCam.get_up_general(f, w, h, el, roll, cx, cy)).max() < 1e-12
-        assert np.abs(op.get_lat_general(f, w, h, el, roll, cx, cy) - PanoCam.get_lat_general(f, w, h, el, roll, cx, cy)).max() < 1e-10
+    """Six random cameras (the reference's fields in tests/golden/reference_checks.npz)."""
+    ref = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_checks.npz"))
+    for i, (f, w, h, el, roll, cx, cy) in enumerate(ref["panocam/cases"]):
+        w, h = int(w), int(h)
+        up, lat = (from_byte_planes(ref[f"panocam/{n}{i}"], ref[f"panocam/{n}{i}/shape"]) for n in ("up", "lat"))
+        assert np.abs(op.get_up_general(f, w, h, el, roll, cx, cy) - up).max() < 1e-12
+        assert np.abs(op.get_lat_general(f, w, h, el, roll, cx, cy) - lat).max() < 1e-10
 
 
 def test_closed_form_focal_matches_fsolve_formulation():

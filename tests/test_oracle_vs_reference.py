@@ -1,89 +1,65 @@
-"""CPU, build container only: the oracle against the imported, unmodified reference (skipped where
-/root/reference is absent, e.g. on the GPU box).  This is the live version of the golden fixtures."""
+"""CPU: the oracle against what the unmodified reference computed for the same inputs, stored under tests/golden/ by
+tests/golden/make_golden_reference_checks.py: its state-dict layout, merged configuration and model-zoo entry per version
+(reference_config.json.gz), and its outputs on seeded synthetic checkpoints and images (reference_checks.npz)."""
+import gzip
+import hashlib
+import json
 import os
-import tempfile
 
+import numpy as np
 import pytest
-import torch
 
+from golden_util import GOLDEN_DIR, compare_result
 from oracle import model as om
 from oracle import weights_gen as wg
-from oracle.ref_shim import reference_available
 from oracle.schema import state_dict_schema
 from oracle.variants import VARIANTS
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not present")
+with gzip.open(os.path.join(GOLDEN_DIR, "reference_config.json.gz"), "rt") as _f:
+    REF_CONFIG = json.load(_f)
+REF = np.load(os.path.join(GOLDEN_DIR, "reference_checks.npz"))
 
 
-@pytest.fixture(scope="module")
-def p2d():
-    th = tempfile.mkdtemp(prefix="pf_ref_")
-    os.environ["TORCH_HOME"] = th
-    os.makedirs(os.path.join(th, "hub", "checkpoints"), exist_ok=True)
-    from oracle.ref_shim import load_reference
-
-    return load_reference(), th
+def _compare(res, prefix, label):
+    compare_result(res, REF, prefix, REF[prefix + "keys"].tolist(), int(REF["stride"]), int(REF["logit_stride"]), 1e-4, label,
+                   edges=bool(REF["edges"]))
 
 
 @pytest.mark.parametrize("version", list(VARIANTS))
-def test_schema_matches_reference(p2d, version):
-    mod, th = p2d
-    sd = {k: torch.zeros(s) for k, s in state_dict_schema(version)}
-    torch.save({"model": sd}, os.path.join(th, "hub", "checkpoints", VARIANTS[version]["ckpt"]))
-    ref_sd = mod.PerspectiveFields(version).state_dict()
-    assert list(ref_sd.keys()) == [k for k, _ in state_dict_schema(version)]
-    for k, s in state_dict_schema(version):
-        assert tuple(ref_sd[k].shape) == tuple(s), k
+def test_schema_matches_reference(version):
+    ref = REF_CONFIG["schema"][version]
+    assert [k for k, _ in ref] == [k for k, _ in state_dict_schema(version)]
+    for (k, s), (_, rs) in zip(state_dict_schema(version), ref):
+        assert tuple(rs) == tuple(s), k
 
 
-def test_live_outputs_match(p2d):
-    mod, th = p2d
+def test_live_outputs_match():
     version = "PersNet_Paramnet-GSV-uncentered"
     sd = wg.synth_state_dict(version, 3)
-    torch.save({"model": sd}, os.path.join(th, "hub", "checkpoints", VARIANTS[version]["ckpt"]))
-    model = mod.PerspectiveFields(version).eval()
     imgs = wg.smooth_images(1, 300, 420, 5)
-    ref = model.inference_batch(imgs)
     ora = om.inference_batch(sd, version, imgs)
-    assert list(ref[0].keys()) == list(ora[0].keys())
-    for k, v in ref[0].items():
-        if isinstance(v, str):
-            continue
-        err = ((v - ora[0][k]).abs().max() / v.abs().max().clamp_min(1e-30)).item()
-        assert err < 1e-4, (k, err)
+    _compare(ora[0], "live/", version)
 
 
-def test_float_input_branch_matches_reference(p2d):
+def test_float_input_branch_matches_reference():
     """perspectivefields.py:47-66: non-uint8 images go through F.interpolate instead of PIL (pins oracle.model.inference_float /
     resize_float, which tests/test_gpu_forward.py uses as the referee for the CUDA float branch)."""
-    import numpy as np
-
-    mod, th = p2d
     version = "Paramnet-360Cities-edina-centered"
     sd = wg.synth_state_dict(version, 0)
-    torch.save({"model": sd}, os.path.join(th, "hub", "checkpoints", VARIANTS[version]["ckpt"]))
-    model = mod.PerspectiveFields(version).eval()
     img = wg.smooth_images(1, 200, 260, 9)[0].astype(np.float32) + 0.25
-    assert np.array_equal(model.aug.apply_image(img), om.resize_float(img, 320, 320))
-    ref = model.inference(img)
-    ora = om.inference_float(sd, version, img)
-    for k, v in ref.items():
-        if isinstance(v, str):
-            continue
-        err = ((v - ora[k]).abs().max() / v.abs().max().clamp_min(1e-30)).item()
-        assert err < 1e-4, (k, err)
+    resized = om.resize_float(img, 320, 320)
+    assert resized.shape == tuple(REF["float/resized/shape"]) and resized.dtype == np.float32
+    assert hashlib.sha256(np.ascontiguousarray(resized).tobytes()).hexdigest() == str(REF["float/resized/sha256"])
+    _compare(om.inference_float(sd, version, img), "float/", version)
 
 
-def test_yaml_configuration_matches_reference(p2d):
+def test_yaml_configuration_matches_reference():
     """perspectivefields_b200/config/*.yaml (defaults + per-variant overrides, parsed with PyYAML) give every inference-relevant
     field the value the reference's yacs tree has after merge_from_file (perspectivefields.py:124-131)."""
     from perspectivefields_b200 import variants as V
 
-    mod, th = p2d
     for version in VARIANTS:
-        sd = {k: torch.zeros(s) for k, s in state_dict_schema(version)}
-        torch.save({"model": sd}, os.path.join(th, "hub", "checkpoints", VARIANTS[version]["ckpt"]))
-        ref = mod.PerspectiveFields(version).cfg
+        ref = REF_CONFIG["cfg"][version]
         mine = V.make_cfg(version)
 
         def walk(a, b, path):
@@ -96,4 +72,4 @@ def test_yaml_configuration_matches_reference(p2d):
                     rv = list(rv) if isinstance(rv, (list, tuple)) else rv
                     assert rv == v, (version, path + k, rv, v)
         walk(mine, ref, "")
-        assert V.model_zoo[version] == mod.perspectivefields.model_zoo[version]
+        assert V.model_zoo[version] == REF_CONFIG["model_zoo"][version]
